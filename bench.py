@@ -5,6 +5,7 @@ random-init weights -> tokens/s for the whole job (BASELINE.json metric).
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the unmodified reference (baseline/_ref) on the same config
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's loss, grad norm, parameters as .npy
 
 Timing: W untimed warm-up steps, then exactly K steps bracketed by barrier + torch.cuda.synchronize(), measured with
 CUDA events on the launching stream, MAX over ranks.  Two timed phases through the SAME public API
@@ -63,7 +64,13 @@ def parse():
     p.add_argument("--graph", type=int, default=-1,
                    help="1/0: replay each micro-batch from a CUDA graph (default: on when one TP group of > 1 GPUs spans "
                         "the job; see host_enqueue_ms_per_step)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step computed to DIR/*.npy (see "
+                        "dump_outputs), so that two builds run with the same arguments can be compared output for output")
+    a = p.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs is implemented for --impl ours only")
+    return a
 
 
 class ClockSampler:
@@ -201,6 +208,35 @@ def megatron_argv(a, n_gpus):
     return argv, vocab
 
 
+DUMP_SAMPLES_PER_TENSOR = 4096
+
+
+def dump_outputs(out_dir, loss, grad_norm, model):
+    """Writes the results of one training step as ``out_dir/<name>.npy``:
+
+    * ``lm_loss.npy`` (float32 [1]): the step's loss, averaged over its micro-batches (absent on ranks that do not
+      compute the loss, i.e. all but the last pipeline stage);
+    * ``grad_norm.npy`` (float32 [1]): the gradient norm before clipping;
+    * ``params_sample.npy`` (float32 [n_tensors, 4096]): every parameter tensor this rank holds after the optimizer
+      update, in ``named_parameters`` order, read at 4096 positions drawn with replacement from a fixed seed: 16 KB per
+      tensor, far below 64 MB in all for every model here.
+
+    The positions depend only on the tensor sizes, so two builds run with the same arguments read the same elements."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    if loss and "lm loss" in loss:
+        np.save(os.path.join(out_dir, "lm_loss.npy"), loss["lm loss"].detach().float().reshape(1).cpu().numpy())
+    np.save(os.path.join(out_dir, "grad_norm.npy"), np.asarray([float(grad_norm)], dtype=np.float32))
+    g = torch.Generator().manual_seed(0)
+    rows = []
+    for m in model:
+        for _, p in m.named_parameters():
+            idx = torch.randint(0, p.numel(), (DUMP_SAMPLES_PER_TENSOR,), generator=g).to(p.device)
+            rows.append(p.detach().reshape(-1)[idx].float().cpu())
+    np.save(os.path.join(out_dir, "params_sample.npy"), torch.stack(rows).numpy())
+
+
 def _fused_tp_active():
     from megatron_llm_b200.parallel import fused_tp
     c = fused_tp.communicator()
@@ -269,8 +305,11 @@ def run_ours(a):
     it_dev = dev_iter() if feeds else None
     it_host = host_iter() if feeds else None
 
+    last_step = {}
+
     def step(it):
         loss, skipped, gnorm, _ = train_step(finetune.forward_step, it, model, optimizer, scheduler)
+        last_step["loss"], last_step["grad_norm"] = loss, gnorm
         return loss
 
     def timed(it, k, read_loss):
@@ -347,6 +386,9 @@ def run_ours(a):
                    "total": round(ex.sum().item(), 3)}
     host_enqueue_ms = timed.host_enqueue_ms
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        # before the e2e phase, which trains on: these are the results of the last step timed in `value`
+        dump_outputs(a.dump_outputs, last_step["loss"], last_step["grad_norm"], model)
     e2e = None
     if not a.no_e2e:
         step(it_host)  # one untimed step on the host-fed path

@@ -146,8 +146,10 @@ def test_selftests_admit_working_kernels_and_reject_broken_ones(fake, monkeypatc
 
 def test_selftest_on_a_cuda_device_runs_in_a_throwaway_process(fake, monkeypatch):
     """On a GPU the first launch of a never-run kernel variant happens in a child process with a time limit: a sticky
-    CUDA error or a dead-locked kernel costs that child, not the job.  Here (no GPU) the child cannot pass -- what is
-    checked is that a crashing child and one that overruns its limit both come back as a clean, loud 'no'."""
+    CUDA error or a dead-locked kernel costs that child, not the job.  Here the child sees no GPU (on a GPU machine too)
+    and cannot pass -- what is checked is that a crashing child and one that overruns its limit both come back as a
+    clean, loud 'no'."""
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")          # read by the child's CUDA start-up; this process uses no device
     monkeypatch.setattr(torch.cuda, "is_current_stream_capturing", lambda: False)
     monkeypatch.setattr(torch.cuda, "current_device", lambda: 0)
     dev = torch.device("cuda", 0)

@@ -161,6 +161,31 @@ def test_bench_presets_build_valid_arguments(monkeypatch):
                                                                         and layout[1] == 1 and not a.recompute)
 
 
+def test_bench_dump_outputs_reads_the_same_positions_every_run(tmp_path):
+    """``bench.py --dump-outputs``: float32 loss, grad norm and a parameter sample whose positions depend only on the
+    tensor sizes, so the files of two runs with the same arguments line up element for element."""
+    import numpy as np
+    import bench
+    torch.manual_seed(0)
+    model = [torch.nn.Sequential(torch.nn.Linear(64, 48), torch.nn.LayerNorm(48)).to(torch.bfloat16)]
+    loss = {"lm loss": torch.tensor(10.5)}
+    bench.dump_outputs(str(tmp_path / "a"), loss, torch.tensor([2.25]), model)
+    bench.dump_outputs(str(tmp_path / "b"), {}, 3.0, model)
+    assert sorted(os.listdir(tmp_path / "a")) == ["grad_norm.npy", "lm_loss.npy", "params_sample.npy"]
+    assert sorted(os.listdir(tmp_path / "b")) == ["grad_norm.npy", "params_sample.npy"]
+    assert np.load(tmp_path / "a" / "lm_loss.npy").tolist() == [10.5]
+    assert np.load(tmp_path / "a" / "grad_norm.npy").dtype == np.float32
+    a, b = np.load(tmp_path / "a" / "params_sample.npy"), np.load(tmp_path / "b" / "params_sample.npy")
+    params = list(model[0].parameters())
+    assert a.dtype == np.float32 and a.shape == (len(params), bench.DUMP_SAMPLES_PER_TENSOR)
+    assert np.array_equal(a, b)
+    for row, p in zip(a, params):       # every sampled value is an element of its tensor; 4096 draws cover 48 elements
+        vals = set(p.detach().float().reshape(-1).tolist())
+        assert set(row.tolist()) <= vals
+        if p.numel() <= 48:
+            assert set(row.tolist()) == vals
+
+
 def test_reference_helper_names_behave():
     """Small public helpers that scripts written against the reference import by name."""
     import os

@@ -6,8 +6,6 @@ import builtins
 import glob
 import os
 
-import pytest
-
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), os.pardir))
 SKIP = (os.sep + "baseline" + os.sep, os.sep + "_build" + os.sep, "gpurun_out", os.sep + ".git" + os.sep)
 
@@ -90,17 +88,31 @@ def test_every_args_attribute_is_a_flag_or_assigned_somewhere(monkeypatch):
 
 def test_build_restores_the_reference_tree_of_the_benchmark_arm(tmp_path, monkeypatch):
     """``baseline/_ref`` (the unmodified reference that ``bench.py --impl reference`` drives) is git-ignored, so a
-    fresh checkout lacks it: ``__graft_entry__.build()`` copies it back, verbatim, and leaves an existing one alone."""
+    fresh checkout lacks it: ``__graft_entry__.build()`` copies the checkout named by ``MLB200_REFERENCE_DIR`` there,
+    verbatim, and leaves an existing one alone.  A small stand-in tree plays the reference checkout."""
     import filecmp
     import __graft_entry__ as entry
-    if not os.path.isdir("/root/reference/megatron"):
-        pytest.skip("no reference checkout on this machine")
-    monkeypatch.setattr(entry, "ROOT", str(tmp_path))
+    src = tmp_path / "Megatron-LLM"
+    for rel, text in [("megatron/__init__.py", ""), ("megatron/training.py", "def pretrain():\n    pass\n"),
+                      ("megatron/core/tensor_parallel/layers.py", "class ColumnParallelLinear:\n    pass\n"),
+                      ("finetune.py", "from megatron.training import pretrain\n"), (".git/HEAD", "ref: main\n"),
+                      ("megatron/__pycache__/training.cpython-312.pyc", "stale")]:
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_text(text)
+    monkeypatch.setattr(entry, "ROOT", str(tmp_path / "repo"))
+    ref = tmp_path / "repo" / "baseline" / "_ref"
+    monkeypatch.delenv("MLB200_REFERENCE_DIR", raising=False)
     entry._ensure_reference_tree()
-    ref = tmp_path / "baseline" / "_ref"
+    assert not ref.exists()
+    monkeypatch.setenv("MLB200_REFERENCE_DIR", str(src))
+    entry._ensure_reference_tree()
     assert (ref / "megatron" / "training.py").is_file() and (ref / "finetune.py").is_file()
-    cmp = filecmp.dircmp("/root/reference/megatron", str(ref / "megatron"), ignore=["__pycache__"])
-    assert not cmp.left_only and not cmp.right_only and not cmp.diff_files
+    assert not (ref / ".git").exists() and not (ref / "megatron" / "__pycache__").exists()
+
+    def same(cmp):
+        return (not cmp.left_only and not cmp.right_only and not cmp.diff_files
+                and all(same(sub) for sub in cmp.subdirs.values()))
+    assert same(filecmp.dircmp(str(src / "megatron"), str(ref / "megatron"), ignore=["__pycache__"]))
     marker = ref / "finetune.py"
     marker.write_text("# kept")
     entry._ensure_reference_tree()
